@@ -2,7 +2,7 @@
 the 8 x 6-block SwinIR, the 23-block RRDBNet and the 28-block SCUNet of configs/inference/*.yaml, random-init weights from
 the seeded generator, on EXACTLY the weights and inputs of the full-config `-m gpu` tests (tests/test_gpu_engines.py):
 
-    python tests/golden/gen_golden_full.py        # needs /root/reference, ~10 min of CPU; writes full_config.npz
+    python tests/golden/gen_golden_full.py        # needs the reference checkout (_ref_import.py), ~10 min of CPU; writes full_config{,_vae,_swinir}.npz
 
 so the chain reference == oracle (tests/test_oracle_golden.py, CPU) and oracle ~ CUDA (GPU) is closed at full width, not
 only at the reduced widths of the other fixtures, and the GPU tests can also be read against the reference directly.
@@ -108,8 +108,11 @@ def main():
     out["scunet_y"] = scu(xc)[..., ::2, ::2].numpy()
     print("scunet full", float(np.abs(out["scunet_y"]).mean()), flush=True)
 
-    np.savez_compressed(OUT / "full_config.npz", **out)
-    print("wrote full_config.npz")
+    # three files, each under 1 MB: the VAE and SwinIR outputs apart from the ControlLDM / RRDBNet / SCUNet ones
+    parts = {"full_config_vae": ("vae",), "full_config_swinir": ("swinir",), "full_config": ("cldm", "rrdb", "scunet")}
+    for name, prefixes in parts.items():
+        np.savez_compressed(OUT / f"{name}.npz", **{k: v for k, v in out.items() if k.startswith(prefixes)})
+        print(f"wrote {name}.npz")
 
 
 if __name__ == "__main__":

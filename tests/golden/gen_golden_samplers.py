@@ -2,7 +2,7 @@
 (diffbir.sampler.{EDMSampler, DPMSolverSampler} and the k_diffusion step functions) with an analytic
 stand-in model on the CPU.
 
-    python tests/golden/gen_golden_samplers.py        # needs /root/reference; writes samplers.npz
+    python tests/golden/gen_golden_samplers.py        # needs the reference checkout (_ref_import.py); writes samplers.npz, samplers_v.npz
 
 tests/test_oracle_golden.py::test_edm_dpm_samplers_match_reference replays the same calls through
 diffbir_b200.sampler and asserts bit equality. The stochastic "SDE" rules need torchsde's Brownian tree
@@ -88,8 +88,11 @@ def main():
             z = fns[solver](den, x0.clone(), s.sigmas, disable=True, eta=HP["eta"], s_noise=HP["s_noise"],
                             noise_sampler=seeded_noise(11))
             out[f"sde_{pname}_{solver}"] = z.numpy()
-    np.savez_compressed(OUT / "samplers.npz", **out)
-    print("wrote", OUT / "samplers.npz", len(out), "arrays")
+    # two files, each under 1 MB: the inputs and eps-parameterization trajectories, and the v-parameterization ones
+    v_keys = [k for k in out if k.startswith(("edm_v_", "edm_sigmas_v", "edm_timesteps_v", "dpm_v_", "sde_v_"))]
+    np.savez_compressed(OUT / "samplers.npz", **{k: v for k, v in out.items() if k not in v_keys})
+    np.savez_compressed(OUT / "samplers_v.npz", **{k: out[k] for k in v_keys})
+    print("wrote", OUT / "samplers.npz", OUT / "samplers_v.npz", len(out), "arrays")
 
 
 if __name__ == "__main__":

@@ -120,7 +120,7 @@ def test_vae_full_config_vs_oracle(golden_dir):
     from diffbir_b200.engine.vae import VaeEngine
     from oracle import cldm as ocl
     no_tf32()
-    g = np.load(golden_dir / "full_config.npz")
+    g = np.load(golden_dir / "full_config_vae.npz")
     sd = make_state_dict(arch.vae_shapes(arch.VAE_CFG), 77)
     eng = VaeEngine(sd, None, "cuda")
     sd_d = to_dev(sd)
@@ -168,7 +168,7 @@ def test_swinir_full_config_vs_oracle(size, golden_dir):
     print(f"swinir {size}: max err / std = {err:.2e}, psnr(peak 1) {psnr(y, ref, 1.0):.1f} dB")
     assert err < 3e-2
     if size == 256:                                            # the reference's own output for this weight / input pair
-        gref = torch.from_numpy(np.load(golden_dir / "full_config.npz")["swinir_y256"]).cuda()
+        gref = torch.from_numpy(np.load(golden_dir / "full_config_swinir.npz")["swinir_y256"]).cuda()
         eg = ((y - gref).abs().max() / gref.std()).item()
         print(f"swinir 256 vs reference fixture: max err / std = {eg:.2e}")
         assert eg < 3e-2

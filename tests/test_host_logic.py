@@ -54,7 +54,7 @@ def test_edm_dpm_samplers_bit_exact_vs_reference(golden_dir):
     src = (golden_dir / "gen_golden_samplers.py").read_text()
     ns = {}
     exec(src[src.index("EDM_CASES = "):src.index("def rnd(")], ns)      # the case tables only (no reference import)
-    g = np.load(golden_dir / "samplers.npz")
+    g = {**np.load(golden_dir / "samplers.npz"), **np.load(golden_dir / "samplers_v.npz")}
     xT = torch.from_numpy(g["xT"])
     cond = dict(c_txt=torch.from_numpy(g["cond_c_txt"]), c_img=torch.from_numpy(g["cond_c_img"]))
     unc = dict(c_txt=torch.from_numpy(g["uncond_c_txt"]), c_img=cond["c_img"].clone())

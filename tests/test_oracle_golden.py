@@ -320,7 +320,7 @@ def test_full_config_oracle_matches_reference(golden_dir):
     GPU tests (tests/golden/gen_golden_full.py): the reference == oracle == CUDA chain is closed at full width too."""
     from oracle import bsrnet as ob
     from oracle import scunet as osc
-    g = np.load(golden_dir / "full_config.npz")
+    g = {k: v for f in ("full_config", "full_config_vae", "full_config_swinir") for k, v in np.load(golden_dir / f"{f}.npz").items()}
     res = {}
     with torch.no_grad():
         usd = make_state_dict(arch.unet_shapes(arch.UNET_CFG), 1234, arch.is_zero_init)
